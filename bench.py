@@ -118,6 +118,22 @@ def build_workload(name, batch):
     return getattr(workloads, builder)(abi.DT_INT8 if dt == "int8" else abi.DT_UINT8, batch=batch, res=res)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, outs):
+    """Write graph output i as <path>/output<i>.npy, its quantised values as float32 (exact).  When all outputs together exceed
+    DUMP_LIMIT_BYTES, each is cut to its share of the limit: a sample of flat indices, seeded by i, in ascending order."""
+    os.makedirs(path, exist_ok=True)
+    total = 4 * sum(o.size for o in outs)
+    for i, o in enumerate(outs):
+        a = o.astype(np.float32)
+        if total > DUMP_LIMIT_BYTES:
+            keep = o.size * DUMP_LIMIT_BYTES // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(i).choice(o.size, keep, replace=False))]
+        np.save(os.path.join(path, f"output{i}.npy"), a)
+
+
 def usable_cpus():
     """CPUs this process may actually use: the affinity mask, capped by the cgroup CPU quota (cpu.max) when one is set."""
     cpus = sorted(os.sched_getaffinity(0))
@@ -319,6 +335,8 @@ def main():
     ap.add_argument("--cpu-window", type=float, default=12.0, help="cpu_baseline: length of the fleet window in seconds; 0 disables")
     ap.add_argument("--pinned", action="store_true", help="e2e with cudaHostAlloc'd caller buffers instead of pageable ones")
     ap.add_argument("--watchdog", type=float, default=780.0, help="seconds after which a stuck run dumps its Python stacks and exits (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the graph outputs of the last timed step to DIR/output<i>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
     if args.watchdog > 0 and int(os.environ.get("RANK", "0")) == 0:
         import faulthandler
@@ -433,6 +451,12 @@ def run_product_arm(args, ngpu, world, barrier):
     wall_dev = time.time() - wall0
     dev_ms = max(sum(a.elapsed_time(b_) for a, b_ in ev[i]) for i in range(ngpu))  # max over GPUs of the K-step device time
     clocks = sampler.finish()
+    if args.dump_outputs:
+        outs = [np.empty(g.dims(o), g.np_dtype) for o in g.outputs]
+        for i, o in enumerate(outs):
+            graph.download(i, o)
+        graph.sync()
+        dump_outputs(args.dump_outputs, outs)
 
     # ---------------- end to end through the reference-facing call with HOST buffers: `e2e` ----------------
     for _ in range(2):

@@ -54,6 +54,9 @@ class FakeGraph:
     def launch(self):
         pass
 
+    def download(self, i, out):
+        out[...] = (np.arange(out.size) % 251).astype(out.dtype).reshape(out.shape)
+
     def sync(self):
         pass
 

@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """Golden vectors for oracle/yolo_post.py: the detection post-processing of the UNMODIFIED examples/tm_yolov3_tiny_uint8.cpp
 (compiled by oracle/build_ref.py into oracle/_ref/libyolo_example.so through oracle/yolo_example_shim.cpp), run on seeded
-quantised head tensors.  Needs /root/reference at build time; the .npz it writes is committed so that the pin holds anywhere.
+quantised head tensors.  Needs the reference tree at build time; the .npz files it writes are committed so that the pin holds
+anywhere.
 usage: make_golden_yolo_post.py [out.npz]"""
 import ctypes as C
 import os
@@ -46,9 +47,16 @@ def run_example(L, q32, s32, z32, q16, s16, z16, prob=0.4, nms=0.25):
     return out[:n].copy()
 
 
+def write_seeded(L, out=os.path.join(HERE, "yolo_example_post_seeded.npz")):
+    """The example's boxes for the heads random_heads() makes from seeds 11 and 12 (tests/test_yolo_post_pinned.py rebuilds the heads)."""
+    np.savez_compressed(out, **{f"boxes_seed{seed}": run_example(L, *random_heads(seed)) for seed in (11, 12)})
+    print("wrote", out)
+
+
 if __name__ == "__main__":
     out = sys.argv[1] if len(sys.argv) > 1 else os.path.join(HERE, "yolo_example_post.npz")
     L = example_lib()
+    write_seeded(L)
     d = {}
     for k, seed in enumerate((5, 6, 7)):
         q32, s32, z32, q16, s16, z16 = random_heads(seed)

@@ -1,5 +1,6 @@
 import json
 import os
+import re
 
 import numpy as np
 
@@ -14,6 +15,63 @@ def load_golden(name):
     g = GraphDef.from_dict(d)
     ref = {int(k[5:]): v for k, v in d.items() if k.startswith("ref_t")}
     return g, d["input"], ref
+
+
+def sha256(a):
+    import hashlib
+
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
+
+
+def seeded_arrays(g):
+    """The arrays of g.to_dict() that the builders derive from numpy seeds alone: weights and weight scales."""
+    return {k: v for k, v in g.to_dict().items() if k.endswith(("_weight", "_weight_scales"))}
+
+
+def seeded_sha256(g):
+    d = seeded_arrays(g)
+    return sha256(np.concatenate([d[k].reshape(-1).view(np.uint8) for k in sorted(d)] or [np.zeros(0, np.uint8)]))
+
+
+class Pin:
+    """A graph pinned to what the reference was run on, plus the reference's outputs, from tests/golden/reference_pins.npz
+    (generator: tests/golden/make_golden_reference_pins.py).  Weights and inputs are rebuilt from their numpy seeds (checked
+    against a digest); scales, zero points and biases come from the file, because the workloads calibrate them with a torch fp32
+    pass whose last bit depends on the host CPU.  A reference tensor is stored as its values, as its SHA-256 digest, or (deep
+    uint8 graphs compared layer by layer) as its difference from the oracle's layer output on the reference's own inputs together
+    with its digest -- rebuilt and checked by layer_by_layer()."""
+
+    _file = None
+
+    def __init__(self, name, g):
+        if Pin._file is None:
+            Pin._file = dict(np.load(os.path.join(GOLDEN, "reference_pins.npz")))
+        d = {k[len(name) + 1:]: v for k, v in Pin._file.items() if k.startswith(name + ".")}
+        assert d, f"{name}: not in reference_pins.npz (run tests/golden/make_golden_reference_pins.py)"
+        assert np.array_equal(seeded_sha256(g), d["seeded_sha256"]), f"{name}: seeded weights differ from the pinned graph"
+        self.graph = GraphDef.from_dict({**d, **seeded_arrays(g)})
+        self.values = {int(k[1:]): v for k, v in d.items() if re.fullmatch(r"t\d+", k)}
+        self.digests = dict(zip(d.get("sha256_ids", []), d.get("sha256", [])))
+        ids = list(d.get("delta_ids", []))
+        sizes = [int(np.prod(self.graph.dims(t))) for t in ids]
+        self.deltas = {t: a.reshape(self.graph.dims(t)) for t, a in zip(ids, np.split(d["delta"], np.cumsum(sizes)[:-1]))} if ids else {}
+
+    def matches(self, t, a):
+        """a equals the reference's tensor t byte for byte."""
+        return np.array_equal(a, self.values[t]) if t in self.values else np.array_equal(sha256(a), self.digests[t])
+
+
+def layer_by_layer(oracle, g, x, pin):
+    """Run every layer of g alone on the reference's tensors (the graph input x, then the reference's output of each earlier
+    layer, rebuilt from `pin` and checked against its digest).  Yields (layer index, the oracle's output, the reference's output)."""
+    ref = {g.inputs[0]: x}
+    for li, L in enumerate(g.layers):
+        h, src = single_layer_graph(g, li)
+        got = oracle.run(h, [ref[t] for t in src])[h.outputs[0]]
+        t = L["output"]
+        ref[t] = (got.astype(np.int32) + pin.deltas[t]).astype(got.dtype)
+        assert pin.matches(t, ref[t]), f"layer {li}: the reference's tensor does not rebuild (the oracle's output for it changed)"
+        yield li, got, ref[t]
 
 
 def quant_u8(x, scale, zp):

@@ -45,6 +45,36 @@ def test_product_arm_control_flow_and_json_contract(monkeypatch, capsys, ngpu, e
     _check_line(json.loads(capsys.readouterr().out.strip().splitlines()[-1]), ngpu, bool(extra))
 
 
+@pytest.mark.parametrize("workload,batch", [("mobilenet_v1_int8", 4), ("yolov5s_int8", 64)])
+def test_dump_outputs_writes_every_graph_output_within_the_limit(monkeypatch, capsys, tmp_path, workload, batch):
+    """--dump-outputs DIR: one float32 .npy per graph output; whole outputs when they fit in 64 MB, else a seeded sample of each
+    (YOLOv5s 640x640 at batch 64 has 4.4 x 10^8 output bytes as float32)."""
+    import numpy as np
+
+    import bench
+    import fake_gpu
+
+    undo = fake_gpu.install()
+    try:
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "2", "--warmup", "0", "--cpu-window", "0", "--watchdog", "0", "--workload", workload,
+                                          "--batch", str(batch), "--dump-outputs", str(tmp_path / "out")])
+        for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
+            monkeypatch.delenv(k, raising=False)
+        bench.main()
+        g, _ = bench.build_workload(workload, batch)
+    finally:
+        undo()
+    capsys.readouterr()
+    files = sorted(os.listdir(tmp_path / "out"))
+    assert files == [f"output{i}.npy" for i in range(len(g.outputs))]
+    dumps = [np.load(tmp_path / "out" / f) for f in files]
+    assert all(a.dtype == np.float32 for a in dumps) and sum(a.nbytes for a in dumps) <= bench.DUMP_LIMIT_BYTES
+    whole = sum(g.numel(t) for t in g.outputs) * 4 <= bench.DUMP_LIMIT_BYTES
+    assert whole == all(a.shape == g.dims(t) for a, t in zip(dumps, g.outputs))
+    if whole:
+        assert np.array_equal(dumps[0], (np.arange(dumps[0].size) % 251).astype(g.np_dtype).reshape(dumps[0].shape))
+
+
 @pytest.mark.parametrize("world", [2, 3])
 def test_torchrun_launch_as_the_driver_does_it(world):
     """python -m torch.distributed.run --nproc-per-node N bench.py --gpus N ... with the stand-ins installed in every rank: rank 0
